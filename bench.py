@@ -3,6 +3,10 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo (torchrun launches it for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm: the oracle port of the reference path
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write what the last timed step computed
+
+With the same arguments every run sees the same inputs (seeded weights, token ids, dropout and mask draws), so the
+files --dump-outputs writes can be compared between two builds of the project.
 
 One "step" = one full optimiser step of the musiclm_small coarse stage (BASELINE.json configs[1]):
 token pre-processing -> embedding gather -> 6 x (attention + conv-FFN) -> logit heads -> CE -> backward ->
@@ -11,6 +15,7 @@ forgetful mask active), batch 16 per GPU, N = 1024 positions, synthetic uniform 
 Prints ONE JSON line (rank 0).
 """
 import argparse
+import atexit
 import json
 import math
 import os
@@ -104,18 +109,29 @@ class ClockSampler:
                                        "-i", str(self.index)], stdout=self.f, stderr=subprocess.DEVNULL)
         except Exception:
             self.p = None
+        atexit.register(self._end)           # the sampler must not outlive a run that fails before stop()
+
+    def _end(self):
+        if self.p is not None:
+            self.p.terminate()
+            try:
+                self.p.wait(timeout=5)
+            except Exception:
+                self.p.kill()
+            self.p = None
+            return True
+        return False
 
     def stop(self):
-        if self.p is None:
-            return dict(sm_mhz=None, sm_max_mhz=None, reasons=["nvidia-smi unavailable"])
-        self.p.terminate()
-        try:
-            self.p.wait(timeout=5)
-        except Exception:
-            self.p.kill()
+        sampled = self._end()
         self.f.flush(); self.f.seek(0)
+        text = self.f.read()
+        self.f.close()
+        os.unlink(self.f.name)
+        if not sampled:
+            return dict(sm_mhz=None, sm_max_mhz=None, reasons=["nvidia-smi unavailable"])
         sm, mx, reasons = [], 0, set()
-        for line in self.f.read().splitlines():
+        for line in text.splitlines():
             c = [x.strip() for x in line.split(",")]
             if len(c) < 9:
                 continue
@@ -288,7 +304,7 @@ def measure(key, args, world, rank, local, inst, full):
     import open_musiclm_b200 as O
     wl = WORKLOADS[key]
     B = args.batch if (full and args.batch) else wl["batch"]
-    steps = args.steps if full else max(5, min(args.steps, 10))
+    steps = args.steps
     torch.manual_seed(0)                                      # identical init on every rank (= the reference's init)
     model = make_model(wl).cuda()
     tr = O.HotPathTrainer(model, cross_entropy_loss_weights=TRAIN["ce_weights"], lr=TRAIN["lr"], lr_warmup=TRAIN["lr_warmup"],
@@ -445,6 +461,8 @@ def run_b200(args):
     inst = Instrument()
     res = measure(args.config, args, world, rank, local, inst, full=True)
     tr = res.pop("tr")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr.loss_out, tr.transformer)
     extras = {}
     del tr
     torch.cuda.empty_cache()
@@ -511,6 +529,22 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, loss, model, n_sample=1 << 22):
+    """What the last timed training step hands its caller: the step's loss (loss.npy) and the updated parameters
+    (parameters.npy: all of them, flattened and concatenated in named_parameters() order; beyond n_sample entries, the
+    entries at a fixed seeded sample of positions, in increasing order).  float32, 16 MB at most."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    with torch.no_grad():
+        flat = torch.cat([p.detach().reshape(-1) for _, p in model.named_parameters()])
+        if flat.numel() > n_sample:
+            idx = torch.randint(0, flat.numel(), (n_sample,), generator=torch.Generator().manual_seed(0)).sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
+        np.save(os.path.join(out_dir, "parameters.npy"), flat.float().cpu().numpy())
+
+
 def cpu_cfg1_forward(cores):
     """BASELINE configs[0]: musiclm_small semantic-stage forward on the host cores, batch 2, N = 256 (oracle port, fp32,
     eval), median of 5 after 2 warm-ups."""
@@ -540,6 +574,9 @@ def main():
     ap.add_argument("--config", default="cfg2", choices=sorted(WORKLOADS), help="headline workload (default: BASELINE configs[1])")
     ap.add_argument("--extra", default="cfg3,cfg4", help="other BASELINE configs timed beside it (sub-results under 'configs'); 'none' to skip")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and a fixed sample of the updated parameters "
+                         "to DIR/*.npy (float32)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -8,9 +8,10 @@ import torch
 
 import open_musiclm_b200 as O
 from open_musiclm_b200 import lib
-from oracle import ref_harness
+from oracle.make_golden_checks import digest
 
 GOLD = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "tiny_*.pt")))
+CHECKS = os.path.join(os.path.dirname(__file__), "golden", "reference_checks.pt")
 
 
 def build_from_fixture(fx):
@@ -45,22 +46,19 @@ def test_state_dict_contract_matches_reference_fixture(path):
 
 
 def test_init_is_bit_identical_to_reference_under_same_seed():
-    if not ref_harness.available():
-        pytest.skip("reference tree not present")
-    ref = ref_harness.import_reference()
-    base = dict(dim=128, depth=2, heads=2, attn_dropout=0.0, ff_dropout=0.1)
-    variants = [dict(), dict(use_conv_ff=False, relative_position_bias_type="t5"),
-                dict(relative_position_bias_type="none", use_absolute_position_embeddings=True)]
-    for extra in variants:
-        kw = dict(base, **extra)
-        for mine, theirs in [(O.create_semantic_transformer, ref.create_semantic_transformer),
-                             (O.create_coarse_transformer, ref.create_coarse_transformer),
-                             (O.create_fine_transformer, ref.create_fine_transformer)]:
-            torch.manual_seed(0); a = mine(**kw).state_dict()
-            torch.manual_seed(0); b = theirs(**kw).state_dict()
-            assert list(a.keys()) == list(b.keys()), extra
-            for k in a:
-                assert torch.equal(a[k], b[k]), (extra, k)
+    """Initial weights under torch.manual_seed(0) against the SHA-256 of the reference's, parameter by parameter
+    (tests/golden/reference_checks.pt, oracle/make_golden_checks.py)."""
+    init = torch.load(CHECKS, weights_only=False)["init"]
+    assert len(init) == 3
+    for case in init:
+        kw = case["kwargs"]
+        for stage, theirs in case["stages"].items():
+            torch.manual_seed(0)
+            a = getattr(O, f"create_{stage}_transformer")(**kw).state_dict()
+            assert [k for k, *_ in theirs] == list(a.keys()), (kw, stage)
+            for k, shape, dtype, sha in theirs:
+                assert tuple(a[k].shape) == shape and str(a[k].dtype) == dtype, (kw, stage, k)
+                assert digest(a[k]) == sha, (kw, stage, k)
 
 
 def test_no_cpu_fallback():

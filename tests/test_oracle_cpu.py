@@ -1,5 +1,5 @@
 """Pins oracle/restatement.py against the golden fixtures produced by the REAL reference
-(oracle/make_golden.py) and, where /root/reference is importable, against the reference live."""
+(oracle/make_golden.py, oracle/make_golden_generate.py, oracle/make_golden_checks.py)."""
 import glob
 import os
 
@@ -7,10 +7,12 @@ import numpy as np
 import pytest
 import torch
 
+import open_musiclm_b200 as O
 from oracle import restatement as R
-from oracle import ref_harness
+from oracle.make_golden_checks import digest
 
 GOLD = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "tiny_*.pt")))
+CHECKS = os.path.join(os.path.dirname(__file__), "golden", "reference_checks.pt")
 
 
 def cfg_from_fixture(fx):
@@ -88,15 +90,10 @@ def test_restatement_optimizer_steps():
 
 
 def test_forgetful_mask_matches_reference():
-    if not ref_harness.available():
-        pytest.skip("reference tree not present")
-    ref_harness.import_reference()
-    import sys
-    utils = sys.modules["open_musiclm.utils"]
-    torch.manual_seed(3)
+    """The reference's utils.generate_mask_with_prob((4, 50), 0.15) after torch.manual_seed(11) is stored in
+    tests/golden/reference_checks.pt."""
+    m_ref = torch.load(CHECKS, weights_only=False)["mask"]
     shape = (4, 50)
-    torch.manual_seed(11)
-    m_ref = utils.generate_mask_with_prob(shape, 0.15, device="cpu")
     torch.manual_seed(11)
     rand = torch.randn(shape)
     m = R.forgetful_mask(shape, 0.15, rand.numpy())
@@ -105,36 +102,27 @@ def test_forgetful_mask_matches_reference():
 
 @pytest.mark.parametrize("stage", ["semantic", "coarse", "fine"])
 def test_restatement_matches_reference_live(stage):
-    """Authoring-container only: mid-size random config, fresh seeds, straight against the reference."""
-    if not ref_harness.available():
-        pytest.skip("reference tree not present")
-    ref = ref_harness.import_reference()
-    common = dict(attn_dropout=0.0, ff_dropout=0.1, grad_shrink_alpha=0.1, non_causal_prefix_size=0,
-                  relative_position_bias_type="continuous", use_memory_efficient_attention=False)
+    """Mid-size random config against what the reference computed for it (tests/golden/reference_checks.pt): its loss
+    and a fixed, seeded sample of its logits, on its own initial weights under torch.manual_seed(5) (rebuilt here with
+    the bit-identical init of this package and checked against the reference's digests)."""
+    fx = torch.load(CHECKS, weights_only=False)["live"][stage]
     torch.manual_seed(5)
-    if stage == "semantic":
-        model = ref.create_semantic_transformer(dim=192, depth=2, heads=3, **common)
-        cfg = R.semantic_cfg(dim=192, depth=2, heads=3, ce_weights=[0.0, 1.0])
-        shapes = [(2, 12), (2, 40)]
-    elif stage == "coarse":
-        model = ref.create_coarse_transformer(dim=192, depth=2, heads=3, num_coarse_quantizers=3, **common)
-        cfg = R.coarse_cfg(dim=192, depth=2, heads=3, ce_weights=[0.0, 0.0, 1.0])
-        shapes = [(2, 12), (2, 20), (2, 9, 3)]
-    else:
-        model = ref.create_fine_transformer(dim=192, depth=2, heads=3, num_coarse_quantizers=3, num_fine_quantizers=5, **common)
-        cfg = R.fine_cfg(dim=192, depth=2, heads=3, ce_weights=[0.0, 0.0, 1.0])
-        shapes = [(2, 12), (2, 5, 3), (2, 5, 5)]
-    wrapper = ref.TokenConditionedTransformerWrapper(transformer=model, unique_consecutive=False,
-                                                     cross_entropy_loss_weights=cfg.ce_weights).eval()
-    g = torch.Generator().manual_seed(99)
-    toks = [torch.randint(0, 1024, s, generator=g) for s in shapes]
-    with torch.no_grad():
-        loss_ref, logits_ref, _ = wrapper(all_token_ids=[t.clone() for t in toks], return_loss=True)
+    model = getattr(O, f"create_{stage}_transformer")(**fx["kwargs"])
     sd = {k: v.detach() for k, v in model.state_dict().items()}
-    loss, logits, *_ = R.loss_and_logits(cfg, sd, [t.numpy() for t in toks])
-    assert abs(float(loss) - float(loss_ref)) / float(loss_ref) < 1e-5
-    for a, b in zip(logits, logits_ref):
-        assert rel(a, b.permute(0, 2, 1)) < 2e-5
+    assert [(k, tuple(v.shape), str(v.dtype), digest(v)) for k, v in sd.items()] == fx["state"]
+    kw = dict(dim=192, depth=2, heads=3, ce_weights=fx["ce_weights"])
+    if stage == "semantic":
+        cfg = R.semantic_cfg(**kw)
+    elif stage == "coarse":
+        cfg = R.coarse_cfg(**kw)
+    else:
+        cfg = R.fine_cfg(**kw)
+    loss, logits, *_ = R.loss_and_logits(cfg, sd, [t.numpy() for t in fx["tokens"]])
+    assert abs(float(loss) - float(fx["loss"])) / float(fx["loss"]) < 1e-5
+    assert len(logits) == len(fx["logits"])
+    for a, b in zip(logits, fx["logits"]):
+        assert tuple(a.shape) == b["shape"]
+        assert rel(a.reshape(-1)[b["index"].long()], b["value"]) < 2e-5
 
 
 GEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "gen_*.pt")))
