@@ -211,21 +211,24 @@ def t5_bucket(relative_position: torch.Tensor, num_buckets=32, max_distance=128)
     return torch.where(is_small, n, val_if_large)
 
 
-def rel_pos_table(sd, n: int, bias_type: str = "continuous", heads: int = 0) -> torch.Tensor:
+def rel_pos_table(sd, n: int, bias_type: str = "continuous", heads: int = 0, dtype=torch.float32) -> torch.Tensor:
     """RelativePositionBias.forward, transformer.py:55-67, restricted to the causal side: returns
     table[h, delta] for delta = i - j in [0, n).  (The reference evaluates the MLP on all 2n-1
     distances and gathers [h, i, j]; entries with j > i are overwritten by the causal mask.)
     't5': T5RelativePositionBias.forward, transformer.py:106-117 (bucket of i - j, see t5_bucket); 'none': zeros
-    (transformer.py:372-373: no bias is added)."""
+    (transformer.py:372-373: no bias is added).  dtype: the precision the table is computed in (float64 for the
+    kernel tests); the parameters are cast to it differentiably."""
     if bias_type == "none":
-        return torch.zeros(heads, n)
+        return torch.zeros(heads, n, dtype=dtype)
     if bias_type == "t5":
-        bucket = t5_bucket(torch.arange(n))                        # delta = i - j >= 0
-        return sd["transformer.rel_pos_bias.relative_attention_bias.weight"][bucket].t().contiguous()
-    x = torch.arange(n, dtype=torch.float32)[:, None]
+        w = sd["transformer.rel_pos_bias.relative_attention_bias.weight"]
+        bucket = t5_bucket(torch.arange(n, device=w.device))       # delta = i - j >= 0
+        return w.to(dtype)[bucket].t().contiguous()
+    p = lambda k: sd[f"transformer.rel_pos_bias.net.{k}"].to(dtype)
+    x = torch.arange(n, dtype=dtype, device=p("0.0.weight").device)[:, None]
     for j in range(3):
-        x = F.silu(x @ sd[f"transformer.rel_pos_bias.net.{j}.0.weight"].t() + sd[f"transformer.rel_pos_bias.net.{j}.0.bias"])
-    x = x @ sd["transformer.rel_pos_bias.net.3.weight"].t() + sd["transformer.rel_pos_bias.net.3.bias"]
+        x = F.silu(x @ p(f"{j}.0.weight").t() + p(f"{j}.0.bias"))
+    x = x @ p("3.weight").t() + p("3.bias")
     return x.t().contiguous()
 
 

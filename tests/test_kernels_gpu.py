@@ -172,11 +172,122 @@ def test_sgemm_small_and_silu(lib):
     zz = z.clone().requires_grad_(True)
     F.silu(zz).backward(dZ)
     out = torch.empty_like(dZ)
-    lib.silu_bwd(dZ, z.contiguous(), out)
+    out_bf = torch.full_like(dZ, float("nan"), dtype=torch.bfloat16)
+    lib.silu_bwd(dZ, z.contiguous(), out, out_bf)
     assert rel(out, zz.grad) < 1e-5
+    assert torch.equal(out_bf, out.bfloat16())
     cs = torch.empty(90, device=DEV)
     lib.colsum(dZ, 90, 1, cs, 300, 90)
     assert rel(cs, dZ.sum(0)) < 1e-5
+    cs0 = torch.randn(90, device=DEV)
+    cs = cs0.clone()
+    lib.colsum(dZ, 90, 1, cs, 300, 90, accumulate=True)
+    assert rel(cs, cs0.double() + dZ.double().sum(0)) < 1e-6
+    # split-K path (accumulate, no activation, no Z, K >= 128, < 64 output tiles): each K slice adds its partial
+    # product into C atomically and only slice 0 adds the bias.  The rel-pos weight-gradient shapes dW4 [h, Hr] =
+    # dY^T a3 and dW0 [Hr, 1] = dz^T x, on top of a non-zero C, against fp64
+    for K in (128, 1000, 2048):
+        for form in ("dW4", "dW0"):
+            if form == "dW4":
+                M, N_ = 8, 512
+                dT = torch.randn(M, K, device=DEV)               # [h, N]
+                a = torch.randn(K, N_, device=DEV)               # [N, Hr]
+                args = (dT, (K, 1), a, (N_, 1))
+                ref = dT.double() @ a.double()
+            else:
+                M, N_ = 512, 1
+                dz = torch.randn(K, M, device=DEV)               # [N, Hr], read transposed
+                x = torch.arange(K, device=DEV, dtype=torch.float32)[:, None] / K
+                args = (dz, (1, M), x, (1, 1))
+                ref = dz.double().t() @ x.double()
+            C0 = torch.randn(M, N_, device=DEV) * float(ref.std())
+            for bias in (None, torch.randn(N_, device=DEV) * float(ref.std())):
+                C = C0.clone()
+                lib.sgemm_small(*args, C, (N_, 1), M, N_, K, bias=bias, accumulate=True)
+                want = ref + C0.double() + (bias.double()[None] if bias is not None else 0)
+                assert rel(C, want) < 1e-5, (K, form, bias is not None, rel(C, want))
+
+
+def test_split3_bias_silu_arange(lib):
+    """The fp32 -> bf16x3 split (bit-exact, both layouts, strided source, grid-stride loop run more than once at the
+    real size N=2048 x Hr=512), the fused bias + SiLU of the hidden layers and the distance ramp."""
+    torch.manual_seed(11)
+    R_, C_ = 2048, 512
+    big = torch.randn(R_, C_ + 40, device=DEV) * torch.exp(2 * torch.randn(R_, C_ + 40, device=DEV))
+    big[0, :4] = torch.tensor([0.0, -0.0, 1e-30, 3e38])
+    for src in (big[:, :C_].contiguous(), big[:, 40:]):
+        hi = src.bfloat16()
+        lo = (src - hi.float()).bfloat16()
+        for weight_mode, order in ((False, (hi, hi, lo)), (True, (hi, lo, hi))):
+            dst = torch.full((R_, 3 * C_), float("nan"), device=DEV, dtype=torch.bfloat16)
+            lib.split3_bf16(src, dst, weight_mode=weight_mode)
+            for j, want in enumerate(order):
+                assert torch.equal(dst[:, j * C_:(j + 1) * C_], want), (weight_mode, j)
+    # the split is what the bf16x3 products rely on: hi + lo reproduces fp32 to ~2^-16 relative
+    src = big[:, :C_]
+    assert rel(src.bfloat16().double() + (src - src.bfloat16().float()).bfloat16().double(), src) < 2 ** -15
+    z0 = torch.randn(R_, C_, device=DEV) * 4
+    bias = torch.randn(C_, device=DEV)
+    z = z0.clone()
+    a = torch.full_like(z, float("nan"))
+    lib.bias_silu(z, bias, a)
+    assert torch.equal(z, z0 + bias)
+    assert rel(a, F.silu(z.double())) < 1e-6
+    for n in (75, 2048, 4097):
+        out = torch.full((n, 1), float("nan"), device=DEV)
+        lib.arange_f32(out)
+        assert torch.equal(out[:, 0], torch.arange(n, device=DEV, dtype=torch.float32))
+
+
+@pytest.mark.parametrize("Hr", [32, 64, 512])
+@pytest.mark.parametrize("N", [75, 1021, 2048])
+def test_bf16x3_gemm_accuracy(lib, Hr, N):
+    """The three bf16x3 product forms of the rel-pos MLP (engine.py _relpos_table / _relpos_backward), fed by
+    split3_bf16, against fp64 of the fp32 operands: forward A3 W3^T; dW += dz^T a over strided [:, :Hr] / [:, 2Hr:]
+    column views with the output as addend; da = dz W in three accumulating calls.  Each must be fp32-class (rel-L2
+    <= 5e-5) AND at least 50x more accurate than the plain bf16 product (hi x hi) of the same operands, which it is
+    only if every lo term is present and in its column block.  Hr = 32 / 64: K below / at the GEMM's 64-wide k-block."""
+    torch.manual_seed(Hr + N)
+    a = F.silu(torch.randn(N, Hr, device=DEV) * 3)
+    w = (torch.rand(Hr, Hr, device=DEV) * 2 - 1) / math.sqrt(Hr)
+    dz = torch.randn(N, Hr, device=DEV)
+    a3 = torch.empty(N, 3 * Hr, device=DEV, dtype=torch.bfloat16)
+    w3 = torch.empty(Hr, 3 * Hr, device=DEV, dtype=torch.bfloat16)
+    dz3 = torch.empty(N, 3 * Hr, device=DEV, dtype=torch.bfloat16)
+    lib.split3_bf16(a, a3)
+    lib.split3_bf16(w, w3, weight_mode=True)
+    lib.split3_bf16(dz, dz3)
+    a_hi, a_lo, dz_hi, dz_lo = a3[:, :Hr], a3[:, 2 * Hr:], dz3[:, :Hr], dz3[:, 2 * Hr:]
+    w_hi, w_lo = w3[:, :Hr], w3[:, Hr:2 * Hr]
+    errs = {}
+    # forward: z = A3 . W3^T (K = 3 Hr), fp32 out
+    ref = a.double() @ w.double().t()
+    z3 = torch.full((N, Hr), float("nan"), device=DEV)
+    z1 = torch.full((N, Hr), float("nan"), device=DEV)
+    lib.gemm(a3, w3, z3, block_n=128)
+    lib.gemm(a_hi, w_hi, z1, block_n=128)
+    errs["fwd"] = (rel(z3, ref), rel(z1, ref))
+    # dW += dz^T a: both operands MN-major, three accumulating products onto a non-zero gradient
+    prod = dz.double().t() @ a.double()
+    g0 = torch.randn(Hr, Hr, device=DEV) * float(prod.std())
+    gw3, gw1 = g0.clone(), g0.clone()
+    for x, y in ((dz_hi, a_hi), (dz_hi, a_lo), (dz_lo, a_hi)):
+        lib.gemm(x, y, gw3, a_mn=True, b_mn=True, M=Hr, N=Hr, K=N, addend=gw3, block_n=128)
+    lib.gemm(dz_hi, a_hi, gw1, a_mn=True, b_mn=True, M=Hr, N=Hr, K=N, addend=gw1, block_n=128)
+    nrm = float(prod.norm())
+    errs["dW"] = (float((gw3.double() - g0.double() - prod).norm()) / nrm, float((gw1.double() - g0.double() - prod).norm()) / nrm)
+    # da = dz W: B MN-major, three calls, the last two accumulating
+    ref = dz.double() @ w.double()
+    da3 = torch.full((N, Hr), float("nan"), device=DEV)
+    da1 = torch.full((N, Hr), float("nan"), device=DEV)
+    lib.gemm(dz_hi, w_hi, da3, b_mn=True, M=N, N=Hr, K=Hr, block_n=128)
+    lib.gemm(dz_hi, w_lo, da3, b_mn=True, M=N, N=Hr, K=Hr, addend=da3, block_n=128)
+    lib.gemm(dz_lo, w_hi, da3, b_mn=True, M=N, N=Hr, K=Hr, addend=da3, block_n=128)
+    lib.gemm(dz_hi, w_hi, da1, b_mn=True, M=N, N=Hr, K=Hr, block_n=128)
+    errs["da"] = (rel(da3, ref), rel(da1, ref))
+    print(f"bf16x3 Hr={Hr} N={N}: " + "  ".join(f"{k} {e3:.2e} (bf16 {e1:.2e})" for k, (e3, e1) in errs.items()))
+    for k, (e3, e1) in errs.items():
+        assert e3 <= 5e-5 and e3 * 50 <= e1, (k, e3, e1)
 
 
 # ------------------------------------------------------------------------------------------------ attention

@@ -2,13 +2,17 @@
 oracle restatement on freshly seeded inputs at the reference's cfg1 size.
 
 Tolerances (north_star / SURVEY 8d): logits rel-L2 <= 1e-2 per returned tensor, loss rel <= 1e-2, every parameter
-gradient cosine >= 0.999 and rel-L2 <= 2e-2, integer path bit-exact.  Two documented exceptions, both in the rel-pos
-bias MLP (DESIGN.md section 4 has the measurements):
+gradient cosine >= 0.999 and rel-L2 <= 2e-2, integer path bit-exact.  The rel-pos bias MLP (DESIGN.md section 4 has
+the measurements):
   * rel_pos_bias.net.3.bias has an analytically ZERO gradient (softmax is invariant to a per-head constant added to its
     bias: sum_j dS_ij = 0); fp32 autograd returns rounding noise (~1e-8), so it is checked in absolute terms.
-  * the other rel-pos MLP parameters receive d(table)[h, i-j] = sum over (batch, i) of dS along a diagonal — a sum of
-    cancelling terms that amplifies the ~1e-2 error every upstream gradient already carries (bf16 backward operands)
-    by the cancellation factor (x4 at N = 1024, x8 at N = 2048, B = 1): cosine >= 0.995, rel-L2 <= 1e-1."""
+  * the other rel-pos MLP parameters receive d(table)[h, i-j] = sum over (batch, i) of dS along a diagonal -- a sum of
+    cancelling terms that amplifies the error of the d(table) the attention backward forms from bf16 operands.  They
+    meet the standard bounds in the fixtures, at cfg1 (N = 256) and in the h = 16 test; only the two real-shape
+    gradient tests pass a looser `relpos` bound to check_grads, set from their B200 measurements (worst rel-L2 /
+    cosine): cfg2 (N = 1024) 4.4e-2 / 0.99912 -> bound 6.5e-2 / 0.9985; cfg3 (N = 2048) 8.1e-2 / 0.99677 -> bound
+    0.1 / 0.995 (the bound before these measurements: 1.5x margin would be looser).  tests/test_relpos_gpu.py shows
+    that this error enters with d(table), not in the MLP backward."""
 import glob
 import os
 
@@ -19,6 +23,7 @@ import torch.nn.functional as F
 
 pytestmark = pytest.mark.gpu
 GOLD = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "tiny_*.pt")))
+RELPOS_STD = (0.999, 2e-2)
 
 
 def rel(a, b):
@@ -39,8 +44,9 @@ def build(fx):
     return m.cuda().eval()
 
 
-def check_grads(got, gold, tag):
-    """Every parameter gradient against the reference's.  Collects all violations before failing, prints the worst."""
+def check_grads(got, gold, tag, relpos=RELPOS_STD):
+    """Every parameter gradient against the reference's.  Collects all violations before failing, prints the worst and
+    every rel-pos gradient.  relpos: (cos_min, rel_max) of the rel-pos MLP parameters (see the module docstring)."""
     bad, worst = [], (1.0, 0.0, "")
     w3 = next((g for k, g in gold.items() if k.endswith("rel_pos_bias.net.3.weight") and g is not None), None)
     for k, g in gold.items():
@@ -58,7 +64,9 @@ def check_grads(got, gold, tag):
             continue
         c, r = cos(mine, g), rel(mine, g)
         worst = min(worst, (c, r, k))
-        c_min, r_max = (0.995, 1e-1) if "rel_pos_bias" in k else (0.999, 2e-2)
+        if "rel_pos_bias" in k:
+            print(tag, k, f"cos {c:.6f} rel-L2 {r:.3e}")
+        c_min, r_max = relpos if "rel_pos_bias" in k else RELPOS_STD
         if not (c >= c_min and r <= r_max):
             bad.append((k, round(c, 5), round(r, 5)))
     print(tag, "worst gradient (cos, rel, name):", worst)
@@ -141,7 +149,8 @@ def test_optimizer_steps_match_reference_fixture():
 
 
 def test_cfg1_semantic_forward_vs_oracle():
-    """BASELINE configs[0]: musiclm_small semantic stage, B=2, N=256, eval; oracle = CPU fp32 restatement."""
+    """BASELINE configs[0]: musiclm_small semantic stage, B=2, N=256, eval; oracle = CPU fp32 restatement.  Logits, loss
+    and every parameter gradient (the SURVEY 8d gradient-check size) with the standard bounds."""
     import open_musiclm_b200 as O
     from oracle import restatement as R
     torch.manual_seed(0)
@@ -162,6 +171,7 @@ def test_cfg1_semantic_forward_vs_oracle():
         r = rel(a, b)
         print("cfg1 logits rel-L2", r)
         assert r <= 1e-2
+    _grads_vs_oracle(m, tr, sd, cfg, toks, "cfg1")
 
 
 def _forward_vs_oracle(model, cfg, toks, ce_w, tag):
@@ -225,7 +235,7 @@ def test_large_arch_heads16_forward_backward_vs_oracle():
 
 
 
-def _grads_vs_oracle(m, tr, sd, cfg, toks, tag):
+def _grads_vs_oracle(m, tr, sd, cfg, toks, tag, relpos=RELPOS_STD):
     from oracle import restatement as R
     names = [k for k, _ in m.named_parameters()]
     sd_g = {k: (v.clone().requires_grad_(True) if k in names else v) for k, v in sd.items()}
@@ -235,7 +245,7 @@ def _grads_vs_oracle(m, tr, sd, cfg, toks, tag):
     tr._micro_batch([t.cuda() for t in toks], False, 0, True)
     got = {k: tr.eng.gview[k] for k in names}
     gold = {k: (sd_g[k].grad if sd_g[k].grad is not None else torch.zeros_like(sd[k])) for k in names}
-    check_grads(got, gold, tag)
+    check_grads(got, gold, tag, relpos)
     tr.eng.arena_g.zero_()
 
 
@@ -252,7 +262,7 @@ def test_cfg2_shape_logits_loss_and_every_gradient_vs_oracle():
             torch.randint(0, 1024, (2, 270, 3), generator=g)]
     cfg = R.coarse_cfg(ce_weights=[0.0, 0.0, 1.0])
     m, tr, sd = _forward_vs_oracle(m, cfg, toks, [0.0, 0.0, 1.0], "cfg2-shape")
-    _grads_vs_oracle(m, tr, sd, cfg, toks, "cfg2-shape")
+    _grads_vs_oracle(m, tr, sd, cfg, toks, "cfg2-shape", relpos=(0.9985, 6.5e-2))
 
 
 def test_cfg3_shape_logits_loss_and_every_gradient_vs_oracle():
@@ -267,7 +277,7 @@ def test_cfg3_shape_logits_loss_and_every_gradient_vs_oracle():
             torch.randint(0, 1024, (1, 1269), generator=g)]
     cfg = R.fine_cfg(ce_weights=[0.0, 0.0, 1.0])
     m, tr, sd = _forward_vs_oracle(m, cfg, toks, [0.0, 0.0, 1.0], "cfg3-shape")
-    _grads_vs_oracle(m, tr, sd, cfg, toks, "cfg3-shape")
+    _grads_vs_oracle(m, tr, sd, cfg, toks, "cfg3-shape", relpos=(0.995, 1e-1))
 
 
 def test_cfg4_musiclm_large_full_depth_forward_vs_oracle():
